@@ -2,13 +2,19 @@
 """bench.py -- CU-Net training-step throughput on B200 (images/sec), with roofline and CPU baseline.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config cunet8|cunet2|cunet16|cunet8bin] [--scaling weak|strong] [--impl reference]
+                    [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  A "step" is one full training step of the reference's train() loop
 (cu-net.py:147-206) on one batch of synthetic input: forward, multi-loss MSE (+ fused landmark decode), backward,
 [gradient allreduce], RMSprop.  `value` times it with the batch already resident in HBM; `e2e` times the same
 step through the public Trainer API with pinned HOST buffers (H2D of image+heatmap and D2H of the loss inside the
 timed region).  `--impl reference` times the reference's own algorithm on the host CPU cores (the oracle port of
-models/cu_net.py -- /root/reference is not present on the GPU box) for the same config and metric.
+models/cu_net.py) for the same config and metric.  `--dump-outputs DIR` writes what the last timed step computed as
+DIR/<name>.npy (see step_outputs); the inputs and initial weights are seeded, so two builds can be compared output
+for output: every timed step starts from the seeded model state (see the resident-input steps in main), so two runs
+give bit-identical heads and landmarks, and loss, gradients and updated weights that differ only by the rounding of
+the floating-point atomics that sum the gradients (RMSprop's first update, g / (sqrt(0.01 g^2) + eps), magnifies that
+rounding on gradients near eps: on a B200 the weights of two runs differed by at most 3e-5 of their largest value).
 """
 import argparse
 import json
@@ -157,6 +163,32 @@ def oracle_loss_main(cfg, batch):
     return 0
 
 
+PROBE_STEPS = 5         # eager steps whose probe-kernel times give the roofline median (not the timed steps)
+DUMP_CAP = 4 << 20      # elements per dumped array: the three large ones stay under 48 MB of float32 together
+
+
+def _sample(flat):
+    """A 1-D device tensor whole, or DUMP_CAP of its elements at fixed seeded positions (the same for equal sizes)."""
+    import torch
+    if flat.numel() <= DUMP_CAP:
+        return flat
+    idx = torch.randint(flat.numel(), (DUMP_CAP,), generator=torch.Generator().manual_seed(0)).sort().values
+    return flat[idx.to(flat.device)]
+
+
+def step_outputs(net, eng):
+    """What the last train_step() handed its caller, as host arrays: the loss it returned (float64), the decoded
+    landmarks and the heads of that step, the model's state_dict after the update (flattened in state_dict order) and
+    the gradients the update used (flattened in parameters() order); the last three are sampled by _sample."""
+    import torch
+    heads = torch.stack([h.float() for h in eng.head_outputs()]).flatten()
+    state = torch.cat([v.detach().float().flatten() for v in net.state_dict().values()])
+    grads = torch.cat([p.grad.float().flatten() for p in net.parameters()])
+    out = dict(loss=eng.loss_value().view(1), preds=eng.preds.float(), heads=_sample(heads), state=_sample(state),
+               grads=_sample(grads))
+    return {k: v.cpu().numpy() for k, v in out.items()}
+
+
 def op_bytes(eng, op, kind):
     """Algorithmic HBM bytes of one launch (DESIGN.md 'Kernels'): every operand read once, every result written once."""
     esz = 2 if eng.tdtype.itemsize == 2 else 4
@@ -209,7 +241,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-loss-check", action="store_true", help="skip the CPU-oracle loss of the first step")
     ap.add_argument("--oracle-loss", action="store_true", help=argparse.SUPPRESS)
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (rank 0, B200 arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     # stdout carries exactly ONE line, the JSON record: anything a library prints there (NCCL writes its version banner
     # to stdout at communicator creation) is sent to stderr instead
     global _OUT_FD
@@ -244,7 +280,7 @@ def main():
         if cfg.get("quant"):
             _emit(dict(impl="reference", unavailable="the CPU reference arm times the full-precision step only"))
             return 0
-        ips, cores = cpu_reference(cfg, args.cpu_sample, max(1, min(args.steps, 3)))
+        ips, cores = cpu_reference(cfg, args.cpu_sample, args.steps, warmup=args.warmup)
         ref_workload = ("CU-Net-%d order %d loss %d, %d classes, 256x256 -> 64x64 heatmaps, train step on the host CPU: "
                         "%d-image sample batch, fp32 (torch CPU), %d threads -- bounded sample of the B200 arm's workload "
                         "(batch %d per GPU, %s)" % (cfg["layer_num"], cfg["order"], cfg["loss_num"], cfg["class_num"],
@@ -255,7 +291,7 @@ def main():
                     config=dict(workload=ref_workload, sample_batch=args.cpu_sample, b200_arm_workload=workload),
                     cpu_baseline=dict(value=ips, unit="images/s", cores=cores, kind="port",
                                       sample="%d-image training step (fwd+MSE+bwd+RMSprop) of the same model, median of %d"
-                                             % (args.cpu_sample, max(1, min(args.steps, 3)))),
+                                             % (args.cpu_sample, args.steps)),
                     e2e=dict(value=ips, unit="images/s", h2d_bytes_per_step=0, d2h_bytes_per_step=0))
         _emit(line)
         return 0
@@ -304,15 +340,27 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
-    def timed(fn, steps):
-        ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    def timed(fn, steps, reset=None):
+        """Device time of ``steps`` calls of fn.  With ``reset``, it is enqueued before every call and each call is
+        bracketed by its own events, so the reset is not timed."""
+        if reset is None:
+            evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))]
+        else:
+            evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
         barrier()
-        ev0.record()
-        for _ in range(steps):
-            fn()
-        ev1.record()
+        if reset is None:
+            evs[0][0].record()
+            for _ in range(steps):
+                fn()
+            evs[0][1].record()
+        else:
+            for ev0, ev1 in evs:
+                reset()
+                ev0.record()
+                fn()
+                ev1.record()
         barrier()
-        ms = ev0.elapsed_time(ev1)
+        ms = sum(ev0.elapsed_time(ev1) for ev0, ev1 in evs)
         if world > 1:
             import torch.distributed as dist
             t = torch.tensor([ms], device=dev)
@@ -320,16 +368,27 @@ def main():
             ms = float(t)
         return ms
 
-    # resident-input steps
+    # resident-input steps.  Every timed step is the same training step: it starts from the seeded initial model state
+    # (Engine.save_state: weights, RMSprop state, BatchNorm running statistics and counters), copied back before it
+    # and outside its timing.  The gradient sums use floating-point atomics, so a step from a given state is reproducible only to
+    # rounding; chained steps would carry that rounding through RMSprop and bf16 activations into outputs that differ
+    # from run to run.  From a fixed state, what the timed steps compute depends on the arguments only.
+    state_init = tr.eng.save_state()
     loss_first = float(tr.train_step())
     for _ in range(args.warmup - 1):
         tr.train_step()
     sampler = ClockSampler(local)
     sampler.start()
-    ms = timed(lambda: tr.train_step(), args.steps)
+    ms = timed(lambda: tr.train_step(), args.steps, reset=lambda: tr.eng.restore_state(state_init))
     sampler.stop_flag = True
     ms_per_step = ms / args.steps
     value = world * B / (ms_per_step / 1000.0)
+    if args.dump_outputs and rank == 0:
+        # before the steps below move the weights on
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in step_outputs(net, tr.eng).items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
 
     # end-to-end steps: pinned host -> device copies and a device -> host read of the loss every step
     loss_host = torch.zeros(1, dtype=torch.float64).pin_memory()
@@ -394,8 +453,7 @@ def main():
             loss_host.copy_(loss.detach().double().view(1), non_blocking=False)
         for _ in range(2):
             module_step()
-        nst = max(2, args.steps // 2)
-        ms_m = timed(module_step, nst) / nst
+        ms_m = timed(module_step, args.steps) / args.steps
         module_api = dict(value=B / (ms_m / 1000.0), unit="images/s", ms_per_step=ms_m,
                           path="net(img); loss.backward(); torch.optim.RMSprop.step() (cu-net.py:171-183), eager launches")
         net.bind_grads()
@@ -417,7 +475,7 @@ def main():
         evs[k] = [torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)]
         eng.probes[id(prm)] = evs[k]
     acc = {k: [] for k in kinds}
-    for _ in range(5):
+    for _ in range(PROBE_STEPS):
         tr._fwd_bwd()
         tr._opt()
         torch.cuda.synchronize()
@@ -481,7 +539,8 @@ def main():
         roofline=dict(bound="hbm", achieved=dom["achieved"], peak=dom["peak"], unit="GB/s", frac=dom["frac"],
                       traffic=traffic, traffic_source=traffic_src, kernel=dom["kernel"], op=dom["op"], us_per_launch=dom["us"],
                       algorithmic_bytes=dom["bytes"], peak_source=pk["source"],
-                      note="probe launches timed eagerly with CUDA events right after the timed region"),
+                      note="probe launches timed eagerly with CUDA events right after the timed region, median of "
+                           "%d steps" % PROBE_STEPS),
         roofline_all=roofs,
         conv_flops=dict(train_gflop_per_image=train_gflop_img, achieved_tflops=tflops,
                         frac_of_bf16_sustained=tflops / pk["tf_sust"], peak_tflops=pk["tf_sust"]),

@@ -462,6 +462,19 @@ class Engine(object):
                                        C.c_void_p(self.lr.data_ptr()), C.c_float(alpha), C.c_float(eps),
                                        L.stream_ptr()), "rmsprop_step")
 
+    def _state(self):
+        return (self.params, self.sq_avg, self.bnbuf, self.counters)
+
+    def save_state(self):
+        """Copy of the model state a training step reads and updates: parameters, optimizer state, BatchNorm running
+        statistics and counters."""
+        return [t.clone() for t in self._state()]
+
+    def restore_state(self, saved):
+        """Put back a save_state() copy (in place, on the current stream: captured graphs keep their buffers)."""
+        for t, k in zip(self._state(), saved):
+            t.copy_(k)
+
     def loss_value(self):
         return self.zbuf[self.loss_off].clone()
 
@@ -589,7 +602,7 @@ class Trainer(object):
         # is a real step on whatever sits in the input buffers: the model state it touches (parameters, optimizer
         # state, BatchNorm running statistics and counters) is put back, so capturing is invisible to training
         e = self.eng
-        keep = [t.clone() for t in (e.params, e.sq_avg, e.bnbuf, e.counters)]
+        keep = e.save_state()
         s = torch.cuda.Stream()
         s.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(s):
@@ -597,8 +610,7 @@ class Trainer(object):
             self._opt()
         torch.cuda.current_stream().wait_stream(s)
         torch.cuda.synchronize()
-        for t, k in zip((e.params, e.sq_avg, e.bnbuf, e.counters), keep):
-            t.copy_(k)
+        e.restore_state(keep)
         del keep
         self._g_fb = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self._g_fb):

@@ -60,11 +60,13 @@ def tiny_case(name, layer_num, order, loss_num, class_num, neck, growth, c0, see
 
 def real_case(name, layer_num, order, loss_num, class_num, n, seed):
     """Real channel configuration (4/32/128): digests only (weights are re-derivable from
-    cunet_oracle.init_state(seed), inputs from synthetic.make_inputs(seed))."""
+    cunet_oracle.init_state(seed), inputs from synthetic.make_inputs(seed)).  Computed in float64: in float32 the
+    small BatchNorm-weight gradients (sums that mostly cancel) move by up to ~2 % with the summation order of the
+    host CPU, so a float32 digest only matches on a machine that sums like the one that recorded it."""
     state = cunet_oracle.init_state(class_num, layer_num, order, seed=seed)
-    net = ref_loader.create_reference_net(class_num, layer_num, order, loss_num)
+    net = ref_loader.create_reference_net(class_num, layer_num, order, loss_num).double()
     missing = net.load_state_dict(state, strict=True)
-    img, hm = synthetic.make_inputs(n, class_num, seed=seed)
+    img, hm = (t.double() for t in synthetic.make_inputs(n, class_num, seed=seed))
     outs, loss = run_reference(net, img, hm, train=True)
     sd = net.state_dict()
     digest = {
@@ -257,8 +259,119 @@ def pylib_case(name):
     torch.save(fx, os.path.join(OUT, name))
 
 
+def history_updates():
+    """The TrainHistory.update() arguments of the checkpoint fixture (shared with tests/test_checkpoint_cpu.py)."""
+    from collections import OrderedDict
+    return [(OrderedDict([("epoch", e)]), OrderedDict([("lr", lr)]),
+             OrderedDict([("train_loss", 1.0 / (e + 1)), ("val_loss", 2.0 / (e + 1))]), OrderedDict([("val_pckh", pck)]))
+            for e, (pck, lr) in enumerate([(0.1, 1e-3), (0.3, 1e-3), (0.2, 5e-4)])]
+
+
+def checkpoint_case(name):
+    """Checkpoint bookkeeping of the REAL reference: TrainHistory (utils/util.py:8-46) over history_updates(), the keys
+    its load_state_dict reads, adjust_lr (utils/util.py:106-119) over 200 epochs, and the parameter trees of its
+    create_cu_net (state_dict names / shapes / dtypes; nn.Conv2d modules in modules() order)."""
+    import contextlib
+    import io
+    import types
+    util = ref_loader.load_reference_util()
+    hist = util["TrainHistory"]()
+    steps = []
+    for args in history_updates():
+        hist.update(*args)
+        steps.append((hist.is_best, hist.best_pckh))
+
+    class Recorder(dict):
+        def __getitem__(self, k):
+            self.read.append(k)
+            return dict.__getitem__(self, k)
+    rec = Recorder(hist.state_dict())
+    rec.read = []
+    util["TrainHistory"]().load_state_dict(rec)
+    opt = types.SimpleNamespace(lr=2.5e-4)
+    optimizer = types.SimpleNamespace(param_groups=[{"lr": 2.5e-4}])
+    lrs = []
+    with contextlib.redirect_stdout(io.StringIO()):
+        for e in range(200):
+            util["adjust_lr"](opt, optimizer, e)
+            lrs.append(opt.lr)
+    net = ref_loader.create_reference_net(5, 3, 1, 2)
+    tree = [(k, tuple(v.shape), v.dtype) for k, v in net.state_dict().items()]
+    net = ref_loader.create_reference_net(5, 3, 2, 3)
+    convs = [(n, tuple(m.weight.shape)) for n, m in net.named_modules() if isinstance(m, nn.Conv2d)]
+    torch.save({"history_steps": steps, "history_state": hist.state_dict(), "history_load_keys": rec.read,
+                "adjust_lr": lrs, "state_tree_C5_L3_K1_loss2": tree, "convs_C5_L3_K2_loss3": convs},
+               os.path.join(OUT, name))
+
+
+def cross_check_inputs():
+    """Seeded inputs of cross_check.pt (tests regenerate them and check the fixture's fingerprint):
+    CU-Net weights (cunet_oracle.init_state) and a batch for class_num 4, layer_num 3, order 1, neck 2, growth 8,
+    16 initial channels; weights and gradients of a four-conv stack for BinOp."""
+    state = cunet_oracle.init_state(4, 3, 1, seed=5, neck_size=2, growth_rate=8, init_chan_num=16)
+    gen = torch.Generator().manual_seed(6)
+    img, hm = torch.rand(2, 3, 64, 64, generator=gen), torch.rand(2, 4, 16, 16, generator=gen)
+    gen = torch.Generator().manual_seed(77)
+    shapes = [(4, 3, 3, 3), (32, 128, 3, 3), (16, 128, 1, 1), (4, 4, 1, 1)]
+    w0 = [(torch.rand(s, generator=gen) * 2 - 1) * 1.2 for s in shapes]
+    g0 = [torch.randn(s, generator=gen) for s in shapes]
+    return dict(state=state, img=img, heatmap=hm, binop_w0=w0, binop_g0=g0)
+
+
+def input_fingerprint(inp):
+    return torch.stack([t.double().sum() for t in [inp["img"], inp["heatmap"]] + list(inp["state"].values())
+                        + inp["binop_w0"] + inp["binop_g0"]])
+
+
+CROSS_STRIDE = 8      # every 8th element of each gradient / binarised weight is stored (the file stays small)
+
+
+def cross_check_case(name):
+    """Outputs of the REAL reference on inputs the other fixtures do not cover: loss and gradients of a CU-Net with
+    three losses (models/cu_net.py), BinOp (models/cu_net_prev_version.py:17-92) on a four-conv stack, and the
+    validation path (pylib/Evaluation.py, HumanAug.GetTransform) on pylib_inputs(seed=23)."""
+    import numpy as np
+    inp = cross_check_inputs()
+    net = ref_loader.create_reference_net(4, 3, 1, 3, neck_size=2, growth_rate=8, init_chan_num=16).double()
+    net.load_state_dict(inp["state"], strict=True)
+    _, loss = run_reference(net, inp["img"].double(), inp["heatmap"].double(), train=True)     # float64: see real_case
+    names = [k for k, _ in net.named_parameters()]
+    grads = torch.cat([p.grad.flatten()[::CROSS_STRIDE] for _, p in net.named_parameters()])
+    BinOp = ref_loader.load_reference_binop()
+    convs = [nn.Conv2d(w.shape[1], w.shape[0], w.shape[2], bias=False) for w in inp["binop_w0"]]
+    for m, w in zip(convs, inp["binop_w0"]):
+        m.weight.data = w.clone()
+    with warnings.catch_warnings():
+        warnings.simplefilter("ignore")
+        op = BinOp(nn.Sequential(*convs))
+        op.binarization()
+        wb = [m.weight.data.flatten()[::CROSS_STRIDE].clone() for m in convs]
+        for m, g in zip(convs, inp["binop_g0"]):
+            m.weight.grad = g.clone()
+        op.restore()
+        op.updateBinaryGradWeight()
+        gb = [m.weight.grad.flatten()[::CROSS_STRIDE].clone() for m in convs]
+    mods = ref_loader.load_reference_pylib()
+    pin = pylib_inputs(seed=23)
+    out, tgt, res = pin["output"], pin["target"], [64, 64]
+    with warnings.catch_warnings():
+        warnings.simplefilter("ignore")
+        pylib = dict(get_preds=mods["Evaluation"].get_preds(out.clone()),
+                     accuracy=mods["Evaluation"].accuracy(out.clone(), tgt.clone(), pin["idxs"]),
+                     final_preds=mods["Evaluation"].final_preds(out.clone(), pin["center"], pin["scale"], res, pin["rot"]),
+                     transform=torch.from_numpy(np.asarray(
+                         mods["HumanAug"].GetTransform(np.array([320.0, 410.0]), 1.7, 30.0, 64, 200), dtype=np.float64)))
+    torch.save({"inputs_fingerprint": input_fingerprint(inp), "stride": CROSS_STRIDE,
+                "cunet_loss": loss.detach(), "cunet_param_names": names, "cunet_grads": grads, "binop_num_targets": op.num_of_params,
+                "binop_wb": wb, "binop_gb": gb,
+                "pylib_fingerprint": torch.stack([out.double().sum(), tgt.double().sum()]), "pylib": pylib},
+               os.path.join(OUT, name))
+
+
 def main():
     os.makedirs(OUT, exist_ok=True)
+    checkpoint_case("checkpoint_ref.pt")
+    cross_check_case("cross_check.pt")
     pylib_case("pylib_eval.pt")
     tiny_case("tiny_L3_K2.pt", 3, 2, 2, 5, 2, 8, 16, seed=11)
     tiny_case("tiny_L2_K1.pt", 2, 1, 2, 3, 4, 8, 16, seed=12)

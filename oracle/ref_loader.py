@@ -1,7 +1,8 @@
 """Execute the real reference sources (build container only).
 
-TEST INFRASTRUCTURE -- see oracle/__init__.py.  /root/reference does not exist on the GPU
-box; everything here raises ``ReferenceUnavailable`` there and callers must skip.
+TEST INFRASTRUCTURE -- see oracle/__init__.py.  Only ``oracle/gen_golden.py`` calls it: the tests compare
+against what it recorded under ``tests/golden/``.  Where the reference tree (``CUNET_REFERENCE_ROOT``) is absent,
+everything here raises ``ReferenceUnavailable``.
 
 Recipe (SURVEY.md Appendix C): ``models/cu_net.py`` is python-2 source; two tokens stop it
 from running under python 3:
@@ -63,6 +64,20 @@ def create_reference_net(class_num, layer_num, order, loss_num,
                                 init_chan_num=init_chan_num, class_num=class_num,
                                 layer_num=layer_num, order=order, loss_num=loss_num)
     return net
+
+
+def load_reference_util():
+    """The REAL ``TrainHistory`` class (utils/util.py:8-46) and ``adjust_lr`` function (utils/util.py:106-119) in one
+    namespace: only their text is executed (the module imports PIL / visdom-era helpers that are irrelevant here)."""
+    if not available():
+        raise ReferenceUnavailable("reference tree not present at %s" % REF_ROOT)
+    from collections import OrderedDict
+    with open(os.path.join(REF_ROOT, "utils", "util.py"), "r") as f:
+        src = f.read()
+    ns = {"OrderedDict": OrderedDict}
+    exec(src[src.index("class TrainHistory():"):src.index("class TrainHistoryFace():")], ns)
+    exec(src[src.index("def adjust_lr(opt, optimizer, epoch):"):src.index("def AdjustLR")], ns)
+    return ns
 
 
 def load_reference_quantize(bits_w, bits_i=8, bits_g=8, exp_dir="/tmp/cunet_ref_exp"):

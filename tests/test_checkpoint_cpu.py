@@ -2,11 +2,10 @@
 the parameter tree of cunet_b200's CUNetB200 carries the reference's names and NCHW shapes, so a state_dict written
 by the reference's DataParallel-wrapped net loads by name, and files written here load in the reference."""
 import os
+from collections import OrderedDict
 
 import pytest
 import torch
-
-from oracle import ref_loader
 
 
 def _History(lr=2.5e-4, epoch=3):
@@ -19,63 +18,55 @@ def _History(lr=2.5e-4, epoch=3):
     return h
 
 
-def _reference_train_history_class():
-    """The REAL TrainHistory class (utils/util.py:8-46): only the class text is executed (the module imports PIL /
-    visdom-era helpers that are irrelevant here)."""
-    from collections import OrderedDict
-    src = open(os.path.join(ref_loader.REF_ROOT, "utils", "util.py")).read()
-    start, end = src.index("class TrainHistory():"), src.index("class TrainHistoryFace():")
-    ns = {"OrderedDict": OrderedDict}
-    exec(src[start:end], ns)
-    return ns["TrainHistory"]
+def _reference(golden_dir):
+    """What the reference's own code recorded (oracle/gen_golden.checkpoint_case): TrainHistory bookkeeping, the keys
+    its load_state_dict reads, adjust_lr over 200 epochs, and the parameter trees of its create_cu_net."""
+    return torch.load(os.path.join(golden_dir, "checkpoint_ref.pt"), weights_only=False)
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present")
-def test_train_history_round_trips_with_the_reference_class(tmp_path):
+def test_train_history_round_trips_with_the_reference_class(tmp_path, golden_dir):
     """A checkpoint's 'train_history' written here loads in the reference's TrainHistory.load_state_dict
     (utils/util.py:40-46: epoch, lr, loss, pckh, best_pckh, is_best) and vice versa, with identical bookkeeping."""
-    from collections import OrderedDict
     from cunet_b200.utils.util import TrainHistory
-    Ref = _reference_train_history_class()
-    ours, ref = TrainHistory(), Ref()
-    for e, (pck, lr) in enumerate([(0.1, 1e-3), (0.3, 1e-3), (0.2, 5e-4)]):
-        args = (OrderedDict([("epoch", e)]), OrderedDict([("lr", lr)]),
-                OrderedDict([("train_loss", 1.0 / (e + 1)), ("val_loss", 2.0 / (e + 1))]), OrderedDict([("val_pckh", pck)]))
+    from oracle import gen_golden
+    ref = _reference(golden_dir)
+    ours = TrainHistory()
+    for args, (is_best, best_pckh) in zip(gen_golden.history_updates(), ref["history_steps"]):
         ours.update(*args)
-        ref.update(*args)
-        assert ours.is_best == ref.is_best and ours.best_pckh == ref.best_pckh
-    assert list(ours.state_dict().keys()) == list(ref.state_dict().keys())
-    assert ours.state_dict() == ref.state_dict()
+        assert ours.is_best == is_best and ours.best_pckh == best_pckh
+    assert list(ours.state_dict().keys()) == list(ref["history_state"].keys())
+    assert ours.state_dict() == ref["history_state"]
     path = str(tmp_path / "h.pt")
     torch.save({"train_history": ours.state_dict()}, path)
-    back = Ref()
-    back.load_state_dict(torch.load(path, weights_only=False)["train_history"])        # KeyError before this round
-    assert back.state_dict() == ref.state_dict()
+    back = torch.load(path, weights_only=False)["train_history"]
+    assert {k: back[k] for k in ref["history_load_keys"]} == {k: ref["history_state"][k] for k in ref["history_load_keys"]}
     mine = TrainHistory()
-    mine.load_state_dict(ref.state_dict())
+    mine.load_state_dict(ref["history_state"])
     assert mine.state_dict() == ours.state_dict() and mine.last_epoch() == 2
     assert TrainHistory().last_epoch() == -1                                            # empty: no sentinel records
 
 
-def _nets(class_num=5, layer_num=3, order=1, loss_num=2):
+def _nets(golden_dir):
+    """Ours and the reference's state_dict (zeros, in the reference's names / order / shapes / dtypes) for class_num 5,
+    layer_num 3, order 1, loss_num 2."""
     from cunet_b200.models.cu_net import create_cu_net
-    ours = create_cu_net(4, 32, 128, class_num, layer_num, order, loss_num)
-    ref = ref_loader.create_reference_net(class_num, layer_num, order, loss_num)
-    return ours, ref
+    ours = create_cu_net(4, 32, 128, 5, 3, 1, 2)
+    ref_sd = OrderedDict((k, torch.zeros(shape, dtype=dt)) for k, shape, dt in _reference(golden_dir)["state_tree_C5_L3_K1_loss2"])
+    return ours, ref_sd
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present")
-def test_reference_checkpoint_loads_by_name(tmp_path):
+def test_reference_checkpoint_loads_by_name(tmp_path, golden_dir):
     from cunet_b200.utils.checkpoint import Checkpoint
-    ours, ref = _nets()
-    ref_sd = ref.state_dict()
+    ours, ref_sd = _nets(golden_dir)
     assert list(ref_sd.keys()) == list(ours.state_dict().keys())          # names and registration order
     # what the reference writes: DataParallel-prefixed keys + RMSprop state (cu-net.py:59-61, utils/checkpoint.py:16-19)
     torch.manual_seed(1)
     for v in ref_sd.values():
         if v.dtype.is_floating_point:
             v.copy_(torch.randn_like(v))
-    opt = torch.optim.RMSprop(ref.parameters(), lr=1e-3, alpha=0.99, eps=1e-8)
+    params = [torch.nn.Parameter(v) for k, v in ref_sd.items() if not k.endswith(("running_mean", "running_var",
+                                                                                  "num_batches_tracked"))]
+    opt = torch.optim.RMSprop(params, lr=1e-3, alpha=0.99, eps=1e-8)
     path = str(tmp_path / "lr-0.001-7")
     torch.save({"train_history": {"lr": [{"lr": 1e-3}], "epoch": [{"epoch": 7}]},
                 "state_dict": {"module." + k: v for k, v in ref_sd.items()},
@@ -89,10 +80,9 @@ def test_reference_checkpoint_loads_by_name(tmp_path):
         assert torch.equal(v, ref_sd[k]), k
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present")
-def test_our_checkpoint_loads_in_the_reference(tmp_path):
+def test_our_checkpoint_loads_in_the_reference(tmp_path, golden_dir):
     from cunet_b200.utils.checkpoint import Checkpoint
-    ours, ref = _nets()
+    ours, ref_sd = _nets(golden_dir)
     ck = Checkpoint()
     ck.save_prefix = str(tmp_path) + os.sep
     opt = torch.optim.RMSprop(ours.parameters(), lr=2.5e-4, alpha=0.99, eps=1e-8)
@@ -101,12 +91,13 @@ def test_our_checkpoint_loads_in_the_reference(tmp_path):
     saved = torch.load(path, weights_only=False)
     assert all(k.startswith("module.") for k in saved["state_dict"])
     # the reference's own loop (utils/checkpoint.py:53-61) on its DataParallel-named dict
-    net_dict = {"module." + k: v for k, v in ref.state_dict().items()}
+    net_dict = {"module." + k: v for k, v in ref_sd.items()}
     for name, param in saved["state_dict"].items():
         assert name in net_dict, name
+        assert param.shape == net_dict[name].shape and param.dtype == net_dict[name].dtype, name
         net_dict[name].copy_(param)
     for k, v in ours.state_dict().items():
-        assert torch.equal(ref.state_dict()[k], v), k
+        assert torch.equal(ref_sd[k], v), k
 
 
 def test_old_checkpoints_without_num_batches_tracked(tmp_path):
@@ -152,8 +143,8 @@ def test_entry_point_resume(tmp_path):
         assert torch.equal(v, a.state_dict()[k]), k
 
 
-def test_lr_schedule_matches_reference():
-    """cu-net.py::adjust_lr == utils/util.py:106-119 (x0.2 at epoch 101, x0.5 at 141 and 161), executed side by side."""
+def test_lr_schedule_matches_reference(golden_dir):
+    """cu-net.py::adjust_lr == utils/util.py:106-119 (x0.2 at epoch 101, x0.5 at 141 and 161), as the reference computed it."""
     import importlib.util
     import types
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -164,30 +155,15 @@ def test_lr_schedule_matches_reference():
     lrs = [entry.adjust_lr(ours, e) for e in range(200)]
     assert lrs[100] == 2.5e-4 and abs(lrs[101] - 5e-5) < 1e-18 and abs(lrs[141] - 2.5e-5) < 1e-18 \
         and abs(lrs[199] - 1.25e-5) < 1e-18
-    if ref_loader.available():
-        import contextlib
-        import io
-        src = open(os.path.join(ref_loader.REF_ROOT, "utils", "util.py")).read()
-        start = src.index("def adjust_lr(opt, optimizer, epoch):")
-        ns = {}
-        exec(src[start:src.index("def AdjustLR")], ns)                 # the function only (the module imports visdom etc.)
-        ref_opt = types.SimpleNamespace(lr=2.5e-4)
-        fake = types.SimpleNamespace(param_groups=[{"lr": 2.5e-4}])
-        with contextlib.redirect_stdout(io.StringIO()):
-            for e in range(200):
-                ns["adjust_lr"](ref_opt, fake, e)
-                assert abs(ref_opt.lr - lrs[e]) < 1e-18, e
+    assert lrs == _reference(golden_dir)["adjust_lr"]
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present")
-def test_quantizer_target_convs_match_reference_module_order():
+def test_quantizer_target_convs_match_reference_module_order(golden_dir):
     """QuanOp / BinOp pick nn.Conv2d modules by their modules()-index (utils/quantize.py:80-102): the parameter tree
     must enumerate its convs in the reference's order (features, hg, linears, intermedia -- models/cu_net.py:299-320)."""
     import torch.nn as nn
-    ours, ref = _nets(class_num=5, layer_num=3, order=2, loss_num=3)
-    conv_names = lambda net: [n for n, m in net.named_modules() if isinstance(m, nn.Conv2d)]   # noqa: E731
-    a, b = conv_names(ours), conv_names(ref)
-    assert a == b and len(a) > 10
-    assert a[0] == "features.conv0" and a[-1].startswith("intermedia.adapters.")
-    shapes = lambda net: [tuple(m.weight.shape) for m in net.modules() if isinstance(m, nn.Conv2d)]   # noqa: E731
-    assert shapes(ours) == shapes(ref)
+    from cunet_b200.models.cu_net import create_cu_net
+    ours = create_cu_net(4, 32, 128, 5, 3, 2, 3)
+    convs = [(n, tuple(m.weight.shape)) for n, m in ours.named_modules() if isinstance(m, nn.Conv2d)]
+    assert convs == _reference(golden_dir)["convs_C5_L3_K2_loss3"] and len(convs) > 10
+    assert convs[0][0] == "features.conv0" and convs[-1][0].startswith("intermedia.adapters.")

@@ -1,15 +1,15 @@
 """Pins the CPU oracle (oracle/*.py) to the reference's own behaviour.
 
-Fixtures in tests/golden/ were produced by the REAL reference (oracle/gen_golden.py).  In the
-build container the real reference module is additionally executed side by side.
+Fixtures in tests/golden/ were produced by the REAL reference (oracle/gen_golden.py); the tests need only them.
+The ``*_live_against_reference`` tests keep their names from when they executed the reference side by side: they now
+compare against its outputs recorded in tests/golden/cross_check.pt, and nothing here runs the reference.
 """
 import os
-import warnings
 
 import pytest
 import torch
 
-from oracle import cunet_oracle, quantize_oracle, evaluation_oracle, ref_loader, synthetic
+from oracle import cunet_oracle, quantize_oracle, evaluation_oracle, synthetic
 
 TINY = ["tiny_L3_K2.pt", "tiny_L2_K1.pt", "tiny_L3_K0.pt"]
 
@@ -67,9 +67,12 @@ def test_oracle_real_config_digest(golden_dir):
     assert list(state.keys()) == fx["state_keys"]
     assert [tuple(v.shape) for v in state.values()] == fx["state_shapes"]
     assert len(state) == 396                                      # SURVEY.md §8(b)
-    net = cunet_oracle.OracleCUNet(state, cfg["class_num"], cfg["layer_num"], cfg["order"],
-                                   cfg["loss_num"])
-    img, hm = synthetic.make_inputs(cfg["n"], cfg["class_num"], seed=cfg["seed"])
+    # float64 on both sides (oracle/gen_golden.real_case): the comparison does not depend on the CPU's summation order
+    net = cunet_oracle.OracleCUNet({k: v.double() if v.is_floating_point() else v for k, v in state.items()},
+                                   cfg["class_num"], cfg["layer_num"], cfg["order"], cfg["loss_num"])
+    for n in net.param_names:
+        net.state[n] = net.state[n].detach().double().requires_grad_(True)
+    img, hm = (t.double() for t in synthetic.make_inputs(cfg["n"], cfg["class_num"], seed=cfg["seed"]))
     outs = net(img)
     loss = cunet_oracle.multi_loss_mse(outs, hm)
     loss.backward()
@@ -84,25 +87,33 @@ def test_oracle_real_config_digest(golden_dir):
         assert int(net.state[k]) == r, k
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree only in build container")
-def test_oracle_against_live_reference():
-    torch.manual_seed(5)
-    ref = ref_loader.create_reference_net(4, 3, 1, 3, neck_size=2, growth_rate=8, init_chan_num=16)
-    net = cunet_oracle.OracleCUNet(ref.state_dict(), 4, 3, 1, 3, neck_size=2, growth_rate=8,
-                                   init_chan_num=16)
-    img = torch.rand(2, 3, 64, 64)
-    hm = torch.rand(2, 4, 16, 16)
-    with warnings.catch_warnings():
-        warnings.simplefilter("ignore")
-        ro = ref(img)
-        rl = cunet_oracle.multi_loss_mse(ro, hm)
-        rl.backward()
-    oo = net(img)
-    ol = cunet_oracle.multi_loss_mse(oo, hm)
+def _cross_check_fixture(golden_dir):
+    from oracle import gen_golden
+    fx = torch.load(os.path.join(golden_dir, "cross_check.pt"), weights_only=False)
+    inp = gen_golden.cross_check_inputs()
+    assert torch.allclose(gen_golden.input_fingerprint(inp), fx["inputs_fingerprint"], rtol=0, atol=1e-9), \
+        "seeded inputs drifted from the fixture's"
+    return fx, inp
+
+
+def test_oracle_against_live_reference(golden_dir):
+    """Loss and gradients of the oracle against the reference's (tests/golden/cross_check.pt, float64) on a
+    configuration none of the other fixtures has: order 1, three losses, neck 2, growth 8, 16 initial channels."""
+    fx, inp = _cross_check_fixture(golden_dir)
+    net = cunet_oracle.OracleCUNet({k: v.double() if v.is_floating_point() else v for k, v in inp["state"].items()},
+                                   4, 3, 1, 3, neck_size=2, growth_rate=8, init_chan_num=16)
+    for n in net.param_names:                      # float64 on both sides, like test_oracle_real_config_digest
+        net.state[n] = net.state[n].detach().double().requires_grad_(True)
+    ol = cunet_oracle.multi_loss_mse(net(inp["img"].double()), inp["heatmap"].double())
     ol.backward()
-    assert _close(ol.detach(), rl.detach())
-    for (k, p) in ref.named_parameters():
-        assert _close(net.state[k].grad, p.grad, 2e-4), k
+    assert _close(ol.detach(), fx["cunet_loss"])
+    assert net.param_names == fx["cunet_param_names"]
+    at = 0
+    for n in net.param_names:
+        g = net.state[n].grad.flatten()[::fx["stride"]]
+        assert _close(g, fx["cunet_grads"][at:at + g.numel()], 2e-4), n
+        at += g.numel()
+    assert at == fx["cunet_grads"].numel()
 
 
 @pytest.mark.parametrize("bits_w", [1, 2, 8])
@@ -148,29 +159,20 @@ def test_binop_oracle_matches_reference_fixture(golden_dir):
         assert _close(gb[j], fx["gb"][i], 1e-4), i
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present (GPU box)")
-def test_binop_oracle_live_against_reference():
-    import torch.nn as nn
-    BinOp = ref_loader.load_reference_binop()
-    gen = torch.Generator().manual_seed(77)
-    convs = [nn.Conv2d(ci, co, k, bias=False) for co, ci, k in ((4, 3, 3), (32, 128, 3), (16, 128, 1), (4, 4, 1))]
-    for m in convs:
-        m.weight.data = (torch.rand(m.weight.shape, generator=gen) * 2 - 1) * 1.2
-    w0 = [m.weight.data.clone() for m in convs]
-    with warnings.catch_warnings():
-        warnings.simplefilter("ignore")
-        op = BinOp(nn.Sequential(*convs))
-        op.binarization()
-        wb, saved = quantize_oracle.binop_binarization(w0[1:3])
-        for a, m in zip(wb, convs[1:3]):
-            assert _close(a, m.weight.data, 1e-6)
-        g0 = [torch.randn(m.weight.shape, generator=gen) for m in convs]
-        for m, g in zip(convs, g0):
-            m.weight.grad = g.clone()
-        op.restore()
-        op.updateBinaryGradWeight()
-    for a, m in zip(quantize_oracle.binop_update_grad(saved, g0[1:3]), convs[1:3]):
-        assert _close(a, m.weight.grad, 1e-4)
+def test_binop_oracle_live_against_reference(golden_dir):
+    """oracle/quantize_oracle.binop_* against the REAL BinOp's binarised weights and fixed gradients on a second conv
+    stack (tests/golden/cross_check.pt)."""
+    fx, inp = _cross_check_fixture(golden_dir)
+    w0, g0, k = inp["binop_w0"], inp["binop_g0"], fx["stride"]
+    idx = quantize_oracle.target_indices(len(w0))
+    assert idx == [1, 2] and len(idx) == fx["binop_num_targets"]
+    wb, saved = quantize_oracle.binop_binarization([w0[i] for i in idx])
+    for a, i in zip(wb, idx):
+        assert _close(a.flatten()[::k], fx["binop_wb"][i], 1e-6), i
+    for a, i in zip(quantize_oracle.binop_update_grad(saved, [g0[i] for i in idx]), idx):
+        assert _close(a.flatten()[::k], fx["binop_gb"][i], 1e-4), i
+    for i in (0, 3):                               # first / last conv untouched
+        assert torch.equal(w0[i].flatten()[::k], fx["binop_wb"][i]) and torch.equal(g0[i].flatten()[::k], fx["binop_gb"][i])
 
 
 @pytest.mark.parametrize("cfg", [(2, 16), (8, 16), (8, 68)])
@@ -292,20 +294,20 @@ def test_product_validation_dropins_match_reference_fixture(golden_dir):
     assert (hm - fx["pts2heatmap"]).abs().max() < 1e-6 and (valid.double() - fx["valid_pts"]).abs().max() < 1e-6
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present")
-def test_evaluation_oracle_live_against_reference():
-    """Side by side with the real pylib modules executed in the build container (different seed than the fixture)."""
+def test_evaluation_oracle_live_against_reference(golden_dir):
+    """The oracle's validation path against the real pylib functions' outputs on a second seed
+    (tests/golden/cross_check.pt; pylib_eval.pt holds the first)."""
     import numpy as np
     from oracle import gen_golden
-    mods = ref_loader.load_reference_pylib()
+    fx = torch.load(os.path.join(golden_dir, "cross_check.pt"), weights_only=False)
+    ref = fx["pylib"]
     inp = gen_golden.pylib_inputs(seed=23)
     out, tgt, res = inp["output"], inp["target"], [64, 64]
-    with warnings.catch_warnings():
-        warnings.simplefilter("ignore")
-        assert torch.equal(evaluation_oracle.get_preds(out), mods["Evaluation"].get_preds(out.clone()))
-        assert torch.allclose(evaluation_oracle.accuracy(out, tgt, inp["idxs"]),
-                              mods["Evaluation"].accuracy(out.clone(), tgt.clone(), inp["idxs"]), atol=1e-7)
-        assert torch.equal(evaluation_oracle.final_preds(out.clone(), inp["center"], inp["scale"], res, inp["rot"]),
-                           mods["Evaluation"].final_preds(out.clone(), inp["center"], inp["scale"], res, inp["rot"]))
-        t_ref = mods["HumanAug"].GetTransform(np.array([320.0, 410.0]), 1.7, 30.0, 64, 200)
-        assert np.abs(evaluation_oracle.get_transform(np.array([320.0, 410.0]), 1.7, 30.0, 64, 200) - t_ref).max() < 1e-12
+    fp = torch.stack([out.double().sum(), tgt.double().sum()])
+    assert torch.allclose(fp, fx["pylib_fingerprint"], rtol=0, atol=1e-9), "seeded inputs drifted from the fixture's"
+    assert torch.equal(evaluation_oracle.get_preds(out), ref["get_preds"])
+    assert torch.allclose(evaluation_oracle.accuracy(out, tgt, inp["idxs"]), ref["accuracy"], atol=1e-7)
+    assert torch.equal(evaluation_oracle.final_preds(out.clone(), inp["center"], inp["scale"], res, inp["rot"]),
+                       ref["final_preds"])
+    t = evaluation_oracle.get_transform(np.array([320.0, 410.0]), 1.7, 30.0, 64, 200)
+    assert np.abs(t - ref["transform"].numpy()).max() < 1e-12

@@ -15,8 +15,10 @@ def test_plan_matches_oracle(cfg):
     plan = plan_mod.Plan(class_num, L, K, loss_num, in_res=64)
     state = cunet_oracle.init_state(class_num, L, K, seed=3)
     gen = torch.Generator().manual_seed(7)
-    img = torch.rand(2, 3, 64, 64, generator=gen)
-    hm = torch.rand(2, class_num, 16, 16, generator=gen)
+    # 4 images: with 2, the BatchNorms of the 1x1 neck normalise over two values, and that ill-conditioning amplifies
+    # float64 rounding into ~1e-4 gradient differences that depend on the host CPU's summation order
+    img = torch.rand(4, 3, 64, 64, generator=gen)
+    hm = torch.rand(4, class_num, 16, 16, generator=gen)
     net = cunet_oracle.OracleCUNet({k: v.double() if v.is_floating_point() else v for k, v in state.items()},
                                    class_num, L, K, loss_num)
     for n in net.param_names:
